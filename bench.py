@@ -149,6 +149,32 @@ def _batch_of(model):
     return int(os.environ.get("ZNICZ_BENCH_BATCH", MODELS[model][0]))
 
 
+DUMP_SAMPLE = 1 << 19    # elements --dump-outputs keeps of a larger array (fixed, seeded sample)
+
+
+def dump_outputs(wf, out_dir):
+    """Writes what the last training step left to the caller: the network output of the last
+    minibatch, the evaluator's error count and every layer's weights and bias, as float32
+    ``<out_dir>/<name>.npy``. An array of more than DUMP_SAMPLE elements is replaced by the
+    same seeded sample of its flattened elements on every run, so no file exceeds 2 MB."""
+    import numpy
+    arrays = {"output": wf.forwards[-1].output}
+    if getattr(wf.evaluator, "n_err", None):
+        arrays["n_err"] = wf.evaluator.n_err
+    for i, f in enumerate(wf.forwards):
+        for attr in ("weights", "bias"):
+            if getattr(f, attr, None):
+                arrays["layer%02d_%s_%s" % (i, f.name, attr)] = getattr(f, attr)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a.map_read()
+        v = numpy.asarray(a.mem, dtype=numpy.float32)
+        if v.size > DUMP_SAMPLE:
+            pick = numpy.random.RandomState(v.size).choice(v.size, DUMP_SAMPLE, replace=False)
+            v = v.ravel()[numpy.sort(pick)]
+        numpy.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def run_arm(args, streaming):
     import torch
     if os.environ.get("ZNICZ_OVERLAP_WGRAD") == "0":        # diagnostic
@@ -202,11 +228,15 @@ def run_arm(args, streaming):
     launches0 = api.counters["launches"]
     t0 = time.perf_counter()
     e0.record()
-    wf.run(iterations=args.steps)
+    n_steps = wf.run(iterations=args.steps)
     e1.record()
     t_enq = time.perf_counter()       # host finished enqueueing (the device may still be busy)
     torch.cuda.synchronize()
     t1 = time.perf_counter()
+    if n_steps != args.steps:
+        raise RuntimeError("the timed region ran %d steps instead of %d" % (n_steps, args.steps))
+    if args.dump_outputs and not streaming and int(os.environ.get("RANK", "0")) == 0:
+        dump_outputs(wf, args.dump_outputs)
     if world > 1:
         dist.barrier()
     clocks = sampler.stop()
@@ -390,7 +420,13 @@ def main():
                          "of the per-GPU batch of the config")
     ap.add_argument("--model", default="cifar_caffe", choices=sorted(MODELS),
                     help="cifar_caffe is the north-star config; the others are extra data points")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one computed (network output, "
+                         "error count, every layer's weights and bias) as DIR/<name>.npy; the "
+                         "inputs are seeded, so runs with the same arguments can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

@@ -1,8 +1,9 @@
-"""Cross-framework golden data: Caffe blob dumps shipped with the reference
-(/root/reference/tests/functional/data/*.txt, read-only test oracles) vs our numpy units —
-the reference's ``tests/functional/test_caffe.py`` strategy (SURVEY §4, "cross-framework golden
-data"). The dump format: ``<name>[\\tnum:N\\tchannels:C\\theight:H\\twidth:W]`` followed by
+"""Cross-framework golden data: Caffe blob dumps shipped with the reference's functional tests
+(``tests/functional/data/*.txt``, stored xz-compressed under tests/golden/caffe) vs our numpy
+units — the reference's ``tests/functional/test_caffe.py`` strategy (SURVEY §4, "cross-framework
+golden data"). The dump format: ``<name>[\\tnum:N\\tchannels:C\\theight:H\\twidth:W]`` followed by
 ``num:i`` / ``channels:c`` headers and H tab-separated rows per channel plane."""
+import lzma
 import os
 
 import numpy
@@ -13,8 +14,8 @@ from veles.znicz_b200.core.memory import Array
 from veles.znicz_b200.core.workflow import DummyWorkflow
 from veles.znicz_b200.ops import conv, gd_conv, gd_pooling, normalization, pooling
 
-DATA = "/root/reference/tests/functional/data"
-pytestmark = pytest.mark.skipif(not os.path.isdir(DATA), reason="reference golden data absent")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+DATA = os.path.join(GOLDEN, "caffe")
 
 
 def read_blob(lines, name, shape=None):
@@ -46,7 +47,7 @@ def read_blob(lines, name, shape=None):
 
 
 def _lines(name):
-    with open(os.path.join(DATA, name)) as f:
+    with lzma.open(os.path.join(DATA, name + ".xz"), "rt") as f:
         return f.readlines()
 
 
@@ -145,18 +146,14 @@ def test_lrn_matches_caffe():
 
 def test_conv3_golden_arrays_forward_and_err_input():
     """The reference ships golden arrays of the CIFAR net's conv3 (5 x 5, pad 2, 32 -> 64 channels,
-    3 images) under tests/data/gd_conv_data (SURVEY Appendix C): forward output and err_input of
-    the numpy oracle against them (relative max error; the arrays come from a Caffe fp32 run)."""
-    import os
-    import numpy
-    import pytest
+    3 images) under tests/data/gd_conv_data (SURVEY Appendix C; copied to tests/golden/gd_conv3):
+    forward output and err_input of the numpy oracle against them (relative max error; the arrays
+    come from a Caffe fp32 run)."""
     from veles.znicz_b200.core.memory import Array
     from veles.znicz_b200.core.workflow import DummyWorkflow
     from veles.znicz_b200.ops import conv, gd_conv
-    base = "/root/reference/tests/data/gd_conv_data/gd_conv3."
-    if not os.path.exists(base + "input.npz"):
-        pytest.skip("reference golden arrays not mounted")
-    x, w, b, y, eo, ei = [numpy.load(base + n + ".npz")["arr_0"] for n in
+    base = os.path.join(GOLDEN, "gd_conv3")
+    x, w, b, y, eo, ei = [numpy.load(os.path.join(base, n + ".npz"))["arr_0"] for n in
                           ("input", "weights", "bias", "output", "err_output", "err_input")]
     wf = DummyWorkflow()
     kw = dict(n_kernels=64, kx=5, ky=5, padding=(2, 2, 2, 2), sliding=(1, 1))
@@ -211,7 +208,7 @@ def _conv_relu(wf, bottom, weights):
 
 
 def test_conv_relu_forward_matches_caffe():
-    """/root/reference/tests/functional/test_caffe.py (conv + ReLU pair, `conv_relu.txt`)."""
+    """The reference's tests/functional/test_caffe.py (conv + ReLU pair, `conv_relu.txt`)."""
     lines = _lines("conv_relu.txt")
     bottom = _read_any(lines, "conv_bottom", (2, 32, 32, 3))
     weights = _read_any(lines, "conv_weights", (2, 5, 5, 3))

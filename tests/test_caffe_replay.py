@@ -1,9 +1,9 @@
 """Whole-iteration replay of a Caffe CIFAR-10 training step, layer by layer
-(/root/reference/tests/functional/test_caffe_complex.py:83-534 on
+(the reference's tests/functional/test_caffe_complex.py:83-534 on
 ``data/cifar_export.tar.xz``; iteration 0 converted by tools/make_caffe_replay.py into
-tests/data/caffe_cifar_iter0.npz, batch 3): every layer gets Caffe's bottom blob / weights /
-top gradient and must reproduce Caffe's top blob / bottom gradient - on the numpy oracle
-(CPU tier) and on the sm_100a path in fp32 and bf16 (GPU tier)."""
+tests/golden/caffe_cifar_iter0/<layer>.<direction>.npz, batch 3): every layer gets Caffe's
+bottom blob / weights / top gradient and must reproduce Caffe's top blob / bottom gradient - on
+the numpy oracle (CPU tier) and on the sm_100a path in fp32 and bf16 (GPU tier)."""
 import os
 
 import numpy
@@ -15,9 +15,11 @@ from veles.znicz_b200.core.workflow import DummyWorkflow
 from veles.znicz_b200.ops import (activation, all2all, conv, gd, gd_conv, gd_pooling,
                                   normalization, pooling)
 
-NPZ = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data", "caffe_cifar_iter0.npz")
-D = numpy.load(NPZ) if os.path.isfile(NPZ) else None
-pytestmark = pytest.mark.skipif(D is None, reason="tests/data/caffe_cifar_iter0.npz missing")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "caffe_cifar_iter0")
+D = {}
+for _f in sorted(os.listdir(GOLDEN)):
+    with numpy.load(os.path.join(GOLDEN, _f)) as _z:
+        D.update((k, _z[k]) for k in _z.files)
 
 CONVS = {"conv1": 32, "conv2": 32, "conv3": 64}
 POOLS = {"pool1": pooling.MaxPooling, "pool2": pooling.AvgPooling, "pool3": pooling.AvgPooling}

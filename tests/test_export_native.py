@@ -117,11 +117,12 @@ def test_native_cpp_test_binary(tmp_path):
     assert "0 failures" in r.stdout and "functional cpu" in r.stdout
 
 
+# the MNIST workflow package of the reference's libZnicz tests (tests/workflow_files/mnist.zip)
+REF_PKG = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "libznicz_mnist.zip")
+
+
 def test_native_loads_reference_package():
-    ref = "/root/reference/libZnicz/tests/workflow_files/mnist.zip"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not mounted")
-    eng = native.NativeEngine(ref)
+    eng = native.NativeEngine(REF_PKG)
     assert eng.num_units == 2
     y = eng.run(numpy.zeros((2, 784), numpy.float32))
     assert y.shape == (2, 10) and abs(float(y.sum()) - 2.0) < 1e-4
@@ -172,10 +173,8 @@ def test_cpu_only_cmake_configuration_builds_and_runs(tmp_path):
     r = subprocess.run(["ctest", "--test-dir", build, "--output-on-failure"], capture_output=True,
                        text=True, timeout=300)
     assert r.returncode == 0, r.stdout[-2000:]
-    ref_pkg = "/root/reference/libZnicz/tests/workflow_files/mnist.zip"
-    if os.path.exists(ref_pkg):
-        numpy.zeros((2, 784), numpy.float32).tofile(tmp_path / "x.f32")
-        r = subprocess.run([os.path.join(build, "znicz_infer"), ref_pkg, str(tmp_path / "x.f32"),
-                            "2", "1", "1", "784"], capture_output=True, text=True, timeout=120)
-        assert r.returncode == 0, r.stderr[-1000:]
-        assert "output 2x1x1x10" in r.stdout, r.stdout
+    numpy.zeros((2, 784), numpy.float32).tofile(tmp_path / "x.f32")
+    r = subprocess.run([os.path.join(build, "znicz_infer"), REF_PKG, str(tmp_path / "x.f32"),
+                        "2", "1", "1", "784"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 0, r.stderr[-1000:]
+    assert "output 2x1x1x10" in r.stdout, r.stdout

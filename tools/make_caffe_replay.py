@@ -1,17 +1,20 @@
 """Converts ONE iteration of the reference's Caffe CIFAR export
-(/root/reference/tests/functional/data/cifar_export.tar.xz: text dumps of every layer's blobs
-before/after its forward and backward pass, batch 3) into a compact ``.npz`` that travels with
-the repo (the tarball is 65 MB of text and only exists where the reference is mounted).
-Arrays are NHWC float32; weights keep Caffe's [F][C][ky][kx] order."""
+(``tests/functional/data/cifar_export.tar.xz`` of the reference tree: text dumps of every layer's
+blobs before/after its forward and backward pass, batch 3) into compact ``.npz`` files that travel
+with the repo, one per layer and direction (the tarball is 65 MB of text).
+Arrays are NHWC float32; weights keep Caffe's [F][C][ky][kx] order.
+
+    python tools/make_caffe_replay.py <reference tree> [iteration]
+"""
+import collections
 import os
 import sys
 import tarfile
 
 import numpy
 
-SRC = "/root/reference/tests/functional/data/cifar_export.tar.xz"
-OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "data",
-                   "caffe_cifar_iter%d.npz")
+OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden",
+                   "caffe_cifar_iter%d")
 
 
 def parse(text):
@@ -41,9 +44,10 @@ def parse(text):
     return blobs
 
 
-def main(iteration=0):
+def main(ref_tree, iteration=0):
     out = {}
-    with tarfile.open(SRC, "r:xz") as tar:
+    src = os.path.join(ref_tree, "tests", "functional", "data", "cifar_export.tar.xz")
+    with tarfile.open(src, "r:xz") as tar:
         for m in tar.getmembers():
             parts = m.name.split("/")
             if len(parts) != 3 or parts[1] != str(iteration):
@@ -60,11 +64,16 @@ def main(iteration=0):
                 else:
                     val = numpy.ascontiguousarray(arr.transpose(0, 2, 3, 1))   # NCHW -> NHWC
                 out["%s/%s/%s" % (layer, direction, name)] = val.astype(numpy.float32)
+    parts = collections.defaultdict(dict)
+    for key, val in out.items():
+        layer, direction, _ = key.split("/")
+        parts[layer + "." + direction][key] = val
     path = OUT % iteration
-    os.makedirs(os.path.dirname(path), exist_ok=True)
-    numpy.savez_compressed(path, **out)
-    print(path, os.path.getsize(path), sorted(out)[:6], len(out))
+    os.makedirs(path, exist_ok=True)
+    for name, arrays in sorted(parts.items()):
+        numpy.savez_compressed(os.path.join(path, name + ".npz"), **arrays)
+    print(path, len(parts), "files", len(out), "arrays")
 
 
 if __name__ == "__main__":
-    main(int(sys.argv[1]) if len(sys.argv) > 1 else 0)
+    main(sys.argv[1], int(sys.argv[2]) if len(sys.argv) > 2 else 0)

@@ -60,6 +60,13 @@ class DataParallel(object):
             import datetime
             kw["timeout"] = datetime.timedelta(seconds=float(os.environ.get(
                 "ZNICZ_DP_TIMEOUT_S", root.common.engine.get("dp_timeout_s", 600))))
+            attempt = int(os.environ.get("TORCHELASTIC_RESTART_COUNT", "0"))
+            if attempt > 0:
+                # torchrun gives a restarted group the rendezvous store of the failed attempt,
+                # which still holds the dead ranks' process-group keys (gloo peer addresses):
+                # a peer reading one connects to a closed port. Keep each attempt's keys apart.
+                store, _, _ = next(dist.rendezvous("env://", rank, ws, timeout=kw["timeout"]))
+                kw["store"] = dist.PrefixStore("attempt%d/" % attempt, store)
             dist.init_process_group(backend=backend, rank=rank, world_size=ws, **kw)
         return cls(device, rank, ws)
 
