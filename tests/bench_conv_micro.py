@@ -1,6 +1,6 @@
 """Micro-benchmark of the tcgen05 conv kernels on the CIFAR shapes (CUDA events, L2 flushed by a
 256 MB write between timed launches). Run on a B200:
-    python tests/bench_conv_micro.py            # ZNICZ_UMMA_DBG / _DEEP / _MT select experiments
+    python tests/bench_conv_micro.py
 """
 import os
 import sys
@@ -54,7 +54,6 @@ for name, n, h, w, c, f, k, pad in SHAPES:
     t_w = timeit(lambda: ext.conv_wgrad(eo, x, parts, splits, g, False, 1, None))
     fl = 2.0 * n * h * w * kw * f / 1e6           # MFLOP; / us = TFLOP/s
     print("%s fprop %.1f us (%.0f TF)  dgrad %.1f us (%.0f TF)  wgrad %.1f us (%.0f TF, splits %d)  "
-          "im2col_tma=%s dbg=%s mt=%s" % (
+          "im2col_tma=%s" % (
               name, t_f, fl / t_f, t_d, fl / t_d if t_d else 0, t_w, fl / t_w, splits,
-              os.environ.get("ZNICZ_IM2COL_TMA", "1"), os.environ.get("ZNICZ_UMMA_DBG", "0"),
-              os.environ.get("ZNICZ_UMMA_MT", "1")))
+              os.environ.get("ZNICZ_IM2COL_TMA", "1")))

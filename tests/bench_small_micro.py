@@ -57,7 +57,6 @@ def conv_case(n, h, w, c, f, k):
         n, h, w, c, f, k, r, timeit(fn), timeit(fn, cold=False)))
 
 
-print("dbg=%s" % os.environ.get("ZNICZ_UMMA_DBG", "0"))
 gemm_case(6, 791, 1392)
 gemm_case(6, 792, 1392)
 gemm_case(6, 792, 128)

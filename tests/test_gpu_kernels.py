@@ -99,6 +99,7 @@ CONV_CASES = [
     (2, 27, 27, 16, 24, 11, 11, (0, 0, 0, 0), (4, 4)),  # AlexNet conv1-like stride 4
     (2, 9, 9, 128, 128, 3, 3, (1, 1, 1, 1), (1, 1)),    # 64-channel slices of one tap (tpk = 1)
     (3, 20, 20, 8, 32, 5, 5, (2, 2, 2, 2), (1, 1)),     # channel-padded first layer (tpk = 8)
+    (40, 32, 32, 8, 32, 5, 5, (2, 2, 2, 2), (1, 1)),   # CIFAR conv1 fprop: 320 CTAs x 4 k-blocks, 3-stage ring
     (2, 10, 10, 16, 16, 3, 3, (1, 1, 1, 1), (1, 1)),    # tpk = 4, dgrad with F = 16
     # TMA im2col operand (C % 64 == 0 fprop / wgrad, F % 64 == 0 stride-1 dgrad)
     (3, 14, 17, 64, 64, 3, 5, (2, 1, 1, 0), (1, 1)),    # asymmetric padding, tiles span images

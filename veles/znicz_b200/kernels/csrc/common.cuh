@@ -17,16 +17,7 @@ namespace zn {
 // carve-up, barrier init, TMEM allocation) and block in pdl_wait() until kernel N has completed
 // and flushed. The ~25 launches of a training step otherwise pay one full drain + launch latency
 // each. ZNICZ_PDL=0 switches the attribute off (plain stream order).
-#ifndef ZN_PDL_EARLY_TRIGGER
-#define ZN_PDL_EARLY_TRIGGER 0
-#endif
-__device__ __forceinline__ void pdl_trigger() {
-#if ZN_PDL_EARLY_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;");
-#endif
-}
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_entry() { pdl_trigger(); pdl_wait(); }
 
 inline bool pdl_enabled() {
   static int on = -1;

@@ -11,7 +11,7 @@ namespace zn {
 template <typename T>
 __global__ void act_forward_k(const T* __restrict__ x, T* __restrict__ y, long long n, int act,
                               float factor) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) stf(y + i, act_fwd(act, ldf(x + i), factor, (int)(i & 1)));
@@ -21,7 +21,7 @@ template <typename T>
 __global__ void act_backward_k(const T* __restrict__ err_y, const T* __restrict__ x,
                                const T* __restrict__ y, T* __restrict__ err_x, long long n,
                                int act, float factor) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) {
@@ -37,7 +37,7 @@ __global__ void act_backward_k(const T* __restrict__ err_y, const T* __restrict_
 template <typename T>
 __global__ void err_act_colsum_k(T* __restrict__ err_y, const T* __restrict__ y, int rows, int cols,
                                  int act, float* __restrict__ partial /*[gridDim.y][cols]*/) {
-  pdl_entry();
+  pdl_wait();
   __shared__ float red[8][33];
   int c = blockIdx.x * 32 + threadIdx.x;
   float acc = 0.f;
@@ -68,7 +68,7 @@ template <typename T>
 __global__ void __launch_bounds__(256) err_act_colsum_vec_k(T* __restrict__ err_y, const T* __restrict__ y,
                                                          int rows, int cols, int act,
                                                          float* __restrict__ partial) {
-  pdl_entry();
+  pdl_wait();
   __shared__ float red[256][9];
   const int groups = cols >> 3;                 // <= 256
   const int lanes = 256 / groups;
@@ -107,7 +107,7 @@ template <typename T>
 __global__ void dropout_forward_k(const T* __restrict__ x, T* __restrict__ y, T* __restrict__ mask,
                                   long long n, const int* __restrict__ rng, uint32_t threshold,
                                   float scale) {
-  pdl_entry();
+  pdl_wait();
   uint32_t seed = (uint32_t)rng[0], counter = (uint32_t)rng[1];
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -120,14 +120,14 @@ __global__ void dropout_forward_k(const T* __restrict__ x, T* __restrict__ y, T*
 
 template <typename T>
 __global__ void mul_k(const T* __restrict__ a, const T* __restrict__ b, T* __restrict__ o, long long n) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) stf(o + i, ldf(a + i) * ldf(b + i));
 }
 template <typename T>
 __global__ void add_k(const T* __restrict__ a, const T* __restrict__ b, T* __restrict__ o, long long n) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) stf(o + i, ldf(a + i) + ldf(b + i));
@@ -136,7 +136,7 @@ template <typename T>
 __global__ void mul_backward_k(const T* __restrict__ x, const T* __restrict__ y,
                                const T* __restrict__ e, T* __restrict__ ex, T* __restrict__ ey,
                                long long n) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) {
@@ -150,7 +150,7 @@ __global__ void mul_backward_k(const T* __restrict__ x, const T* __restrict__ y,
 template <typename T>
 __global__ void axpby_2d_k(const T* __restrict__ src, int src_ld, int soff, T* __restrict__ dst,
                            int dst_ld, int doff, int rows, int len, float alpha, float beta) {
-  pdl_entry();
+  pdl_wait();
   long long n = (long long)rows * len;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -169,7 +169,7 @@ __global__ void axpby_2d_k(const T* __restrict__ src, int src_ld, int soff, T* _
 template <typename T>
 __global__ void swap01_2d_k(const T* __restrict__ src, int src_ld, int soff, T* __restrict__ dst,
                             int dst_ld, int doff, int A, int Bn, int len) {
-  pdl_entry();
+  pdl_wait();
   const long long n = (long long)A * Bn * len;
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride) {
@@ -184,7 +184,7 @@ __global__ void swap01_2d_k(const T* __restrict__ src, int src_ld, int soff, T* 
 template <typename T>
 __global__ void crop_nhwc_k(const T* __restrict__ in, T* __restrict__ out, int N, int H, int W, int C,
                             int oh, int ow, int top, int left, int backward) {
-  pdl_entry();
+  pdl_wait();
   if (!backward) {
     long long n = (long long)N * oh * ow * C;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -213,7 +213,7 @@ __global__ void crop_nhwc_k(const T* __restrict__ in, T* __restrict__ out, int N
 template <typename TS, typename TD>
 __global__ void gather_rows_k(const TS* __restrict__ src, const int* __restrict__ idx,
                               TD* __restrict__ dst, int count, int max_rows, long long row) {
-  pdl_entry();
+  pdl_wait();
   long long n = (long long)max_rows * row;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
@@ -226,7 +226,7 @@ __global__ void gather_rows_k(const TS* __restrict__ src, const int* __restrict_
 }
 __global__ void gather_labels_k(const int* __restrict__ src, const int* __restrict__ idx,
                                 int* __restrict__ dst, int count, int max_rows) {
-  pdl_entry();
+  pdl_wait();
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < max_rows) dst[i] = i < count ? src[idx[i]] : -1;
 }
@@ -237,7 +237,7 @@ __global__ void gather_minibatch_k(const TS* __restrict__ src, const int* __rest
                                    const int* __restrict__ hdr, TD* __restrict__ dst,
                                    int* __restrict__ labels_dst, int max_rows, int row8,
                                    TD* __restrict__ dst_pad, int C, int CP) {
-  pdl_entry();
+  pdl_wait();
   const int count = hdr[0];
   const int* idx = hdr + 4;
   const int total = max_rows * row8;
@@ -277,7 +277,7 @@ __global__ void gather_minibatch_k(const TS* __restrict__ src, const int* __rest
 // implicit-GEMM gather can use 16-byte chunks
 template <typename T>
 __global__ void pad_channels_k(const T* __restrict__ x, T* __restrict__ y, int pixels, int C, int CP) {
-  pdl_entry();
+  pdl_wait();
   const int total = pixels * CP;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int p = i / CP, c = i - p * CP;
@@ -289,7 +289,7 @@ __global__ void pad_channels_k(const T* __restrict__ x, T* __restrict__ y, int p
 
 template <typename T>
 __global__ void mask_mul_k(T* __restrict__ w, const T* __restrict__ mask, long long n) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) stf(w + i, ldf(w + i) * ldf(mask + i));
@@ -297,7 +297,7 @@ __global__ void mask_mul_k(T* __restrict__ w, const T* __restrict__ mask, long l
 
 template <typename TS, typename TD>
 __global__ void cast_k(const TS* __restrict__ s, TD* __restrict__ d, long long n) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) stf(d + i, ldf(s + i));
@@ -307,7 +307,7 @@ __global__ void cast_k(const TS* __restrict__ s, TD* __restrict__ d, long long n
 template <typename T>
 __global__ void scatter_offsets_k(const T* __restrict__ in, const int* __restrict__ offs,
                                   T* __restrict__ out, long long n, int accumulate) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < n; i += stride) out[offs[i]] = in[i];
@@ -393,7 +393,7 @@ void launch_gather_rows(const void* src, bool src_bf16, const int* idx, void* ds
 __global__ void pull_from_host_k(const uint4* __restrict__ src, uint4* __restrict__ dst, long long n16,
                                  const unsigned char* __restrict__ src_b, unsigned char* __restrict__ dst_b,
                                  int tail) {
-  pdl_entry();
+  pdl_wait();
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += stride)
     dst[i] = __ldcv(src + i);
@@ -414,7 +414,7 @@ void launch_pull_from_host(const void* src_dev_alias, void* dst, long long nbyte
 template <typename T>
 __global__ void pad_channels_vec_k(const T* __restrict__ x, T* __restrict__ y, long long groups, int C,
                                    int CP8) {
-  pdl_entry();
+  pdl_wait();
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < groups; i += stride) {
     const long long p = i / CP8;
@@ -434,7 +434,7 @@ __global__ void pad_channels_vec_k(const T* __restrict__ x, T* __restrict__ y, l
 // ---- fp8 (e4m3) per-tensor quantisation: q = sat(x * 448 / amax) -------------------------------
 template <typename T>
 __global__ void absmax_k(const T* __restrict__ x, long long n, float* __restrict__ amax) {
-  pdl_entry();
+  pdl_wait();
   float m = 0.f;
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
@@ -445,7 +445,7 @@ __global__ void absmax_k(const T* __restrict__ x, long long n, float* __restrict
 template <typename T>
 __global__ void quant_e4m3_k(const T* __restrict__ x, unsigned char* __restrict__ q, long long n,
                              const float* __restrict__ amax) {
-  pdl_entry();
+  pdl_wait();
   const float scale = 448.f / fmaxf(*amax, 1e-12f);
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
@@ -518,7 +518,7 @@ __global__ void lstm_cell_fwd_k(const float* __restrict__ z, const float* __rest
                                 float* __restrict__ c, float* __restrict__ gates,
                                 T* __restrict__ h_out, long long ldh, T* __restrict__ h_next,
                                 long long ldn, int batch, int H) {
-  pdl_entry();
+  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= batch * H) return;
   const int b = i / H, j = i - b * H;
@@ -545,7 +545,7 @@ __global__ void lstm_cell_bwd_k(const T* __restrict__ err_h, long long lde,
                                 const float* __restrict__ dc_next, const float* __restrict__ gates,
                                 const float* __restrict__ c, const float* __restrict__ c_prev,
                                 float* __restrict__ dc_prev, T* __restrict__ dz, int batch, int H) {
-  pdl_entry();
+  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= batch * H) return;
   const int b = i / H, j = i - b * H;

@@ -32,7 +32,7 @@ __global__ void __launch_bounds__(128)
 fc_small_forward_k(const T* __restrict__ x, const float* __restrict__ w,
                    const float* __restrict__ bias, T* __restrict__ out_t, float* __restrict__ out_f,
                    int* __restrict__ max_idx, int n_in, int n_out, int act, int softmax, EvalArgs ev) {
-  pdl_entry();
+  pdl_wait();
   __shared__ float red[4][FCS_MAX_OUT];
   const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const T* xr = x + (size_t)row * n_in;
@@ -110,7 +110,7 @@ fc_small_backward_k(const T* __restrict__ err, const T* __restrict__ y, const T*
                     const float* __restrict__ w, T* __restrict__ err_in,
                     float* __restrict__ gw_parts, float* __restrict__ gb_parts, int batch, int n_in,
                     int n_out, int act, float alpha, float beta, int need_ei, int need_gw) {
-  pdl_entry();
+  pdl_wait();
   extern __shared__ float s_err[];       // [rows_here][FCS_MAX_OUT]
   const int bs = gridDim.y, part = blockIdx.y;
   const int per = (batch + bs - 1) / bs;

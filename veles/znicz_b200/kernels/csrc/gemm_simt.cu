@@ -76,7 +76,7 @@ struct Epilogue {
 template <typename AL, typename BL>
 __global__ void __launch_bounds__(256) gemm_simt_k(AL A, BL B, Epilogue ep, int M, int N, int K,
                                                    int k_chunk) {
-  pdl_entry();
+  pdl_wait();
   __shared__ float As[16][65];
   __shared__ float Bs[16][65];
   int tx = threadIdx.x % 16, ty = threadIdx.x / 16;

@@ -9,11 +9,13 @@
 //   (im2col of x, or the dgrad gather of err_out) as 16-byte chunks straight into the swizzled
 //   shared-memory tile — no im2col buffer in HBM (the reference unpacks 16 images at a time into
 //   a temp buffer and calls cuBLAS, /root/reference/conv.py:268-297, gd_conv.py:313-423).
+//   A_IM2COL_K: the A_GATHER_K operand fetched by TMA in im2col mode instead (see below).
 //   B_TMA_K   B stored [N][K];  B_TMA_MN  B stored [K][N].
 //
 // Warp roles (192 threads): warps 0-3 = gather producers (if any) then epilogue (TMEM -> regs ->
 // bias/activation/alpha-beta -> global); warp 4 = TMA producer; warp 5 = TMEM allocator + the
-// single thread that issues tcgen05.mma and commits to mbarriers. 4-stage smem ring.
+// single thread that issues tcgen05.mma and commits to mbarriers. 4-stage smem ring (3 stages for
+// short reductions, see launch_cfg).
 //
 // This covers: FC forward (TMA_K x TMA_K, fused bias+activation), FC dgrad (TMA_K x TMA_MN,
 // alpha/beta), FC wgrad (TMA_MN x TMA_MN), conv fprop (GATHER_K x TMA_K, fused bias+act),
@@ -27,16 +29,16 @@ namespace zn {
 
 using namespace umma;
 
-// A_IM2COL_K / A_IM2COL_MN: the same implicit-GEMM operands as A_GATHER_K / A_GATHER_MN, but
-// fetched by TMA in im2col mode (one instruction per [pixels x 64 channels] block instead of a
-// 128-thread LDGSTS gather) - channel counts that are multiples of 64 only.
-enum { A_TMA_K = 0, A_TMA_MN = 1, A_GATHER_K = 2, A_GATHER_MN = 3, A_IM2COL_K = 4, A_IM2COL_MN = 5 };
+// A_IM2COL_K: the same implicit-GEMM operand as A_GATHER_K, but fetched by TMA in im2col mode
+// (one instruction per [128 pixels x 64 channels] block instead of a 128-thread LDGSTS gather) -
+// channel counts that are multiples of 64 only.
+enum { A_TMA_K = 0, A_TMA_MN = 1, A_GATHER_K = 2, A_GATHER_MN = 3, A_IM2COL_K = 4 };
 enum { B_TMA_K = 0, B_TMA_MN = 1 };
 enum { G_NONE = 0, G_IM2COL = 1, G_DGRAD = 2 };
 
 constexpr int BLOCK_M = 128;
 constexpr int BLOCK_K = 64;          // bf16 elements = 128 bytes = one SW128 row
-constexpr int STAGES_DEFAULT = 4;   // deep (8-stage) variant: see launch_cfg
+constexpr int STAGES_DEFAULT = 4;   // 3-stage variant for short reductions: see launch_cfg
 constexpr int A_BYTES = BLOCK_M * 128;
 
 struct ConvGeomU {
@@ -64,13 +66,7 @@ struct GemmParams {
   // gather source
   const __nv_bfloat16* gsrc; ConvGeomU g; int gather_kind;
   int gK;                      // valid extent of the gathered K (fprop/dgrad) or M (wgrad) index
-  // A_GATHER_K only: consecutive 128-row tiles streamed through ONE pipeline per CTA, each with
-  // its own TMEM columns (amortises prologue / epilogue latency for short-K convolutions)
-  int mt;
   int ktab_n;                  // entries of the gather lookup table (dynamic shared memory)
-  int tma_store;               // epilogue: stage the bf16 tile in smem, one TMA store per warp
-  int dbg;                     // experiments: 1 = producers skip the gather, 2 = skip the MMAs,
-                               // 4 = skip the TMA loads, 8 = skip the epilogue stores, 32 = empty kernel
 };
 
 // ---- gather: 8 consecutive "inner" indices of one "pixel" -> 16 bytes ------------------------
@@ -78,7 +74,6 @@ struct GemmParams {
 // vec mode   : ktab[k / 8] = (ky << 24) | (kx << 16) | c0     (16-byte chunks never straddle a tap)
 // scalar mode: ktab[k]     = (ky << 24) | (kx << 16) | c
 constexpr int KTAB = 4096;
-constexpr int MT_MAX = 4;      // tiles streamed through one CTA (TMEM columns: BLOCK_N * mt <= 512)
 
 struct PixCtx { const __nv_bfloat16* base; int y, x, valid; };
 
@@ -289,12 +284,11 @@ __host__ __device__ constexpr int min_ctas() {
 template <int BLOCK_N, int A_MODE, int B_MODE, int GKIND, int GVEC, int STAGES, bool FP8 = false>
 __global__ void __launch_bounds__(192, (min_ctas<BLOCK_N, B_MODE, STAGES>()))
 gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-            const __grid_constant__ CUtensorMap tmap_c, const GemmParams p) {
-  pdl_trigger();
+            const GemmParams p) {
   constexpr int B_BYTES = b_bytes<BLOCK_N, B_MODE>();
   constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   constexpr bool A_GATHER = (A_MODE == A_GATHER_K || A_MODE == A_GATHER_MN);
-  constexpr bool A_MN = (A_MODE == A_TMA_MN || A_MODE == A_GATHER_MN || A_MODE == A_IM2COL_MN);
+  constexpr bool A_MN = (A_MODE == A_TMA_MN || A_MODE == A_GATHER_MN);
   constexpr bool B_MN = (B_MODE == B_TMA_MN);
   constexpr uint32_t TMEM_COLS = BLOCK_N < 32 ? 32 : BLOCK_N;
   constexpr uint32_t IDESC = FP8 ? make_idesc_e4m3(BLOCK_M, BLOCK_N)
@@ -306,7 +300,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[STAGES];
   __shared__ __align__(8) uint64_t empty_bar[STAGES];
-  __shared__ __align__(8) uint64_t tmem_full_bar[MT_MAX];    // one per streamed tile
+  __shared__ __align__(8) uint64_t tmem_full_bar;
   __shared__ uint32_t tmem_base_smem;
 
   // 1024-byte aligned tile area (SWIZZLE_128B atoms are 1024 B)
@@ -318,15 +312,8 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
   int* const ktab = reinterpret_cast<int*>(tiles + (size_t)STAGES * STAGE_BYTES);
   float* const s_bias = reinterpret_cast<float*>(ktab + ((p.ktab_n + 3) & ~3));
 
-  if (p.dbg & 32) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int mt_cfg = (A_MODE == A_GATHER_K && p.mt > 1) ? p.mt : 1;
-  const int m_tiles_total = (p.M + BLOCK_M - 1) / BLOCK_M;
-  const int mtile0 = blockIdx.y * mt_cfg;
-  const int ntiles = min(mt_cfg, m_tiles_total - mtile0);       // tiles this CTA streams (>= 1)
-  const int m0 = mtile0 * BLOCK_M, n0 = blockIdx.x * BLOCK_N;
-  uint32_t tmem_cols = TMEM_COLS;                                 // power of two >= 32
-  while (tmem_cols < (uint32_t)(BLOCK_N * mt_cfg)) tmem_cols <<= 1;
+  const int m0 = blockIdx.y * BLOCK_M, n0 = blockIdx.x * BLOCK_N;
   const int total_kb = (p.K + KBLK - 1) / KBLK;
   const int kb_begin = blockIdx.z * p.k_blocks_per_split;
   const int kb_end = min(total_kb, kb_begin + p.k_blocks_per_split);
@@ -337,7 +324,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
       mbar_init(&full_bar[s], (A_GATHER ? 128u : 0u) + 1u);
       mbar_init(&empty_bar[s], 1u);
     }
-    for (int j = 0; j < MT_MAX; ++j) mbar_init(&tmem_full_bar[j], 1u);
+    mbar_init(&tmem_full_bar, 1u);
     fence_barrier_init();
   }
   if (warp == 4 && lane == 0) {
@@ -345,7 +332,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
     tma_prefetch_desc(&tmap_b);
   }
   if (warp == 5) {
-    tmem_alloc(&tmem_base_smem, tmem_cols);
+    tmem_alloc(&tmem_base_smem, TMEM_COLS);
     tmem_relinquish();
   }
   if (A_GATHER) build_ktab(ktab, p.g, GKIND, p.gK);
@@ -362,33 +349,13 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
   if (warp == 4) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      for (int gi = 0; gi < num_kb * ntiles; ++gi) {
-        const int i = gi % num_kb;
-        const int s = gi % STAGES; const uint32_t ph = (gi / STAGES) & 1;
+      for (int i = 0; i < num_kb; ++i) {
+        const int s = i % STAGES; const uint32_t ph = (i / STAGES) & 1;
         mbar_wait(&empty_bar[s], ph ^ 1);
         uint8_t* sa = tiles + (size_t)s * STAGE_BYTES;
         uint8_t* sb = sa + A_BYTES;
         const int k0 = (kb_begin + i) * KBLK;
-        if (p.dbg & 4) { mbar_arrive(&full_bar[s]); continue; }
-        if (A_MODE == A_IM2COL_MN) {
-          // conv wgrad: tile = [64 pixels (reduction rows)][128 reduction-weight indices] = two
-          // [64 pixels x 64 channels] im2col boxes (one tap each); a block past Kw is skipped
-          const ConvGeomU& g = p.g;
-          const int pix0 = (kb_begin + i) * BLOCK_K;
-          const int q = pix0 % g.OW; const int t2 = pix0 / g.OW;
-          const int pr = t2 % g.OH; const int n = t2 / g.OH;
-          const int w0 = q * g.SX - g.PL, h0 = pr * g.SY - g.PT;
-          const int nblk = (m0 + 64 < p.gK) ? 2 : 1;
-          mbar_arrive_expect_tx(&full_bar[s], (uint32_t)(B_BYTES + nblk * 8192));
-          for (int mb = 0; mb < nblk; ++mb) {
-            const int kidx0 = m0 + mb * 64;
-            const int tap = kidx0 / g.C, c0 = kidx0 - tap * g.C;
-            tma_load_im2col_4d(sa + mb * 8192, &tmap_a, &full_bar[s], c0, w0, h0, n,
-                               (uint16_t)(tap % g.KX), (uint16_t)(tap / g.KX));
-          }
-        } else {
-          mbar_arrive_expect_tx(&full_bar[s], TX_BYTES);
-        }
+        mbar_arrive_expect_tx(&full_bar[s], TX_BYTES);
         if (A_MODE == A_IM2COL_K) {
           // conv fprop / stride-1 dgrad: tile rows = pixels m0 .. m0 + 127, k-block = 64
           // channels of ONE filter tap
@@ -425,10 +392,8 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
   } else if (warp == 5) {
     // ===================== MMA issuer =====================
     if (lane == 0) {
-      for (int gi = 0; gi < num_kb * ntiles; ++gi) {
-        const int i = gi % num_kb;
-        const uint32_t d_tmem = tmem_base + (uint32_t)((gi / num_kb) * BLOCK_N);
-        const int s = gi % STAGES; const uint32_t ph = (gi / STAGES) & 1;
+      for (int i = 0; i < num_kb; ++i) {
+        const int s = i % STAGES; const uint32_t ph = (i / STAGES) & 1;
         mbar_wait(&full_bar[s], ph);
         if (A_GATHER && GVEC == 2) fence_proxy_async_smem();   // LDGSTS data -> async proxy
         tc_fence_after();
@@ -441,43 +406,30 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                                    : make_smem_desc(sa + k * 32, 16, 1024);
           const uint64_t db = B_MN ? make_smem_desc(sb + k * 2048, 8192, 1024)
                                    : make_smem_desc(sb + k * 32, 16, 1024);
-          if (!(p.dbg & 2)) {
-            if (FP8) mma_f8(d_tmem, da, db, IDESC, (i > 0 || k > 0) ? 1u : 0u);
-            else mma_f16(d_tmem, da, db, IDESC, (i > 0 || k > 0) ? 1u : 0u);
-          }
+          if (FP8) mma_f8(tmem_base, da, db, IDESC, (i > 0 || k > 0) ? 1u : 0u);
+          else mma_f16(tmem_base, da, db, IDESC, (i > 0 || k > 0) ? 1u : 0u);
         }
         mma_commit(&empty_bar[s]);          // smem slot reusable once these MMAs retire
-        if (i == num_kb - 1) mma_commit(&tmem_full_bar[gi / num_kb]);   // this tile's accumulator
+        if (i == num_kb - 1) mma_commit(&tmem_full_bar);   // the accumulator is complete
       }
     }
   } else {
-    // ============ gather producers, then epilogue (warps 0-3), software-pipelined ============
-    // Round tt issues the gathers of tile tt and then drains the accumulator of tile tt - 1:
-    // with several tiles streamed through one CTA (GemmParams::mt) the epilogue of a tile
-    // overlaps the MMAs of the next one (up to STAGES k-blocks of operands are already in flight),
-    // and the prologue (barriers, TMEM, lookup table) is paid once.
-#pragma unroll 1
-    for (int tt = 0; tt <= ntiles; ++tt) {
-    if (A_GATHER && tt < ntiles) {
+    // ===================== gather producers (if any), then epilogue (warps 0-3) ================
+    if (A_GATHER) {
       const int t = threadIdx.x;            // 0..127
       if (A_MODE == A_GATHER_K) {
         // tile row r = t is GEMM row m0 + t (a pixel); chunks run over the reduction index
-        {
-        const int tj = tt;
-        const int m = m0 + tj * BLOCK_M + t;
-        const int gbase = tj * num_kb;           // position of this tile in the stage sequence
-        const PixCtx ctx = (GKIND == G_IM2COL) ? decode_out_pixel(p.gsrc, p.g, m, p.M)
-                                               : decode_in_pixel(p.gsrc, p.g, m, p.M);
+        const PixCtx ctx = (GKIND == G_IM2COL) ? decode_out_pixel(p.gsrc, p.g, m0 + t, p.M)
+                                               : decode_in_pixel(p.gsrc, p.g, m0 + t, p.M);
         if (GVEC == 2) {
           // asynchronous gather: issue the LDGSTS of a stage as soon as its slot is free; the
           // stage's full barrier is armed by the copies themselves
 #pragma unroll 1
           for (int i = 0; i < num_kb; ++i) {
-            const int s = (gbase + i) % STAGES; const uint32_t ph = ((gbase + i) / STAGES) & 1;
+            const int s = i % STAGES; const uint32_t ph = (i / STAGES) & 1;
             mbar_wait(&empty_bar[s], ph ^ 1);
             const uint32_t row_base = smem_u32(tiles + (size_t)s * STAGE_BYTES) + t * 128;
-            if (!(p.dbg & 1))
-              gather_row_async<GKIND>(row_base, t & 7, ktab, p.g, ctx, (kb_begin + i) * BLOCK_K);
+            gather_row_async<GKIND>(row_base, t & 7, ktab, p.g, ctx, (kb_begin + i) * BLOCK_K);
             cp_async_mbar_arrive_noinc(&full_bar[s]);
           }
         } else {
@@ -491,7 +443,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
             gather_row<GKIND, GVEC>(nv, ktab, p.g, ctx, k0, p.gK);
           }
           if (i >= 0) {
-            const int s = (gbase + i) % STAGES; const uint32_t ph = ((gbase + i) / STAGES) & 1;
+            const int s = i % STAGES; const uint32_t ph = (i / STAGES) & 1;
             mbar_wait(&empty_bar[s], ph ^ 1);
             uint8_t* sa = tiles + (size_t)s * STAGE_BYTES;
 #pragma unroll
@@ -504,7 +456,6 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
           for (int c8 = 0; c8 < 8; ++c8) v[c8] = nv[c8];
         }
         }
-        }   // tiles of this CTA
       } else {
         // A_GATHER_MN (conv wgrad): tile = [64 reduction rows (pixels)][128 m (kidx)];
         // thread -> reduction row kr = t % 64, 64-wide m block = t / 64 (8 chunks of 8 kidx)
@@ -550,11 +501,9 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
         }
       }
     }
-    // ===================== epilogue of tile tt - 1 =====================
-    if (tt == 0) continue;
-    const int tj = tt - 1;
+    // ===================== epilogue =====================
     if (num_kb > 0) {
-      mbar_wait(&tmem_full_bar[tj], 0);
+      mbar_wait(&tmem_full_bar, 0);
       tc_fence_after();
     }
     // The epilogue runs once per tile, so every instruction of it is an instruction-cache miss:
@@ -562,17 +511,13 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
     // fetch stalls alone. This one is a rolled loop over 8-column chunks - TMEM loads double
     // buffered (the next chunk is in flight while this one is stored) - with the output mode
     // decided once per thread; the loop body is a few hundred instructions, fetched once.
-    enum { EPI_TMA = 0, EPI_BF16 = 1, EPI_RAW_T = 2, EPI_RAW = 3, EPI_SLOW = 4, EPI_NONE = 5,
-           EPI_BIASROW = 6, EPI_F32 = 7 };
-    {
-    const int row = m0 + tj * BLOCK_M + warp * 32 + lane;
+    enum { EPI_BF16, EPI_RAW_T, EPI_RAW, EPI_SLOW, EPI_NONE, EPI_BIASROW, EPI_F32 };
+    const int row = m0 + warp * 32 + lane;
     const bool raw32 = !p.out_bf16 && p.beta == 0.f && p.alpha == 1.f && !p.bias && p.act == 0;
     float* const rbase = reinterpret_cast<float*>(p.out) +
                          (p.split_stride > 0 ? (long long)blockIdx.z * p.split_stride : 0LL);
     int mode;
-    if (p.tma_store) mode = EPI_TMA;
-    else if (row >= p.M || (p.dbg & 8))
-      mode = (p.bias_out && row == p.M && !(p.dbg & 8)) ? EPI_BIASROW : EPI_NONE;
+    if (row >= p.M) mode = (p.bias_out && row == p.M) ? EPI_BIASROW : EPI_NONE;
     else if (p.split_stride == 0 && !p.out_trans && p.out_bf16 && p.beta == 0.f) mode = EPI_BF16;
     else if (p.split_stride == 0 && !p.out_trans && !p.out_bf16 && p.beta == 0.f && !raw32)
       mode = EPI_F32;        // fp32 row-major with bias / activation (LSTM gate pre-activations,
@@ -581,7 +526,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
     else if (raw32 && (p.ldo & 3) == 0 && (reinterpret_cast<uintptr_t>(rbase) & 15) == 0)
       mode = EPI_RAW;
     else mode = EPI_SLOW;
-    const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(tj * BLOCK_N);
+    const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16);
 
     auto emit = [&](const uint32_t (&r)[8], int c0) {
       const int nb = n0 + c0;
@@ -592,7 +537,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
           if (nb + j < p.N) p.bias_out[(long long)blockIdx.z * p.N + nb + j] = __uint_as_float(r[j]);
         return;
       }
-      if (mode == EPI_TMA || mode == EPI_BF16 || mode == EPI_F32) {
+      if (mode == EPI_BF16 || mode == EPI_F32) {
         float v[8];
         {
           const float4 b0 = *reinterpret_cast<const float4*>(s_bias + c0);
@@ -622,8 +567,6 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
             for (int j = 0; j < 8; ++j)
               v[j] = act_fwd5_fast(p.act, fmaf(__uint_as_float(r[j]), p.alpha, v[j]));
         }
-        // bf16 pack: one 16-byte store per 8 outputs. TMA mode stages the 32 x BLOCK_N sub-tile
-        // of this warp in the (idle by now) pipeline buffers; it leaves with one TMA store below
         if (p.dmul != nullptr && mode == EPI_BF16) {
           // err_input *= f'(x): x has the layout of the output (row pitch ldo)
           const __nv_bfloat16* dx = p.dmul + (long long)row * p.ldo + nb;
@@ -650,10 +593,9 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
           }
           return;
         }
-        __nv_bfloat16* q = (mode == EPI_TMA)
-            ? reinterpret_cast<__nv_bfloat16*>(tiles + warp * 8192 + lane * (BLOCK_N * 2)) + c0
-            : reinterpret_cast<__nv_bfloat16*>(p.out) + (long long)row * p.ldo + nb;
-        if (mode == EPI_TMA || (nb + 8 <= p.N && (p.ldo & 7) == 0)) {
+        // bf16 pack: one 16-byte store per 8 outputs
+        __nv_bfloat16* q = reinterpret_cast<__nv_bfloat16*>(p.out) + (long long)row * p.ldo + nb;
+        if (nb + 8 <= p.N && (p.ldo & 7) == 0) {
           st8(q, v);
         } else {                       // ragged last chunk / row pitch not a multiple of 16 bytes
 #pragma unroll
@@ -691,7 +633,7 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
     if (num_kb > 0) tmem_ld_32x8(trow, rb);
 #pragma unroll 1
     for (int c0 = 0; c0 < BLOCK_N; c0 += 8) {
-      if (n0 + c0 >= p.N && mode != EPI_TMA) break;     // chunk beyond the last column
+      if (n0 + c0 >= p.N) break;     // chunk beyond the last column
       if (num_kb > 0) tmem_ld_wait();
 #pragma unroll
       for (int j = 0; j < 8; ++j) ra[j] = rb[j];
@@ -699,24 +641,12 @@ gemm_umma_k(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
       emit(ra, c0);
     }
     if (num_kb > 0) tmem_ld_wait();
-    if (p.tma_store) {
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0 && !(p.dbg & 8)) {
-        // rows / columns beyond M / N are clipped by the tensor map
-        tma_store_2d(&tmap_c, tiles + warp * 8192, n0, m0 + tj * BLOCK_M + warp * 32);
-        tma_store_commit_and_wait_read();
-      }
-      __syncwarp();
-    }
-    }
-    }   // rounds (tiles of this CTA)
     tc_fence_before();
   }
   __syncthreads();
   if (warp == 5) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, tmem_cols);
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -798,20 +728,6 @@ static bool im2col_tma_enabled() {
   return on != 0;
 }
 
-// bf16 output tile map for the TMA-store epilogue: dims {N, M}, box {BN, 32}, no swizzle
-static int make_map_out(CUtensorMap* m, const void* ptr, long long N, long long M, long long ldo, int bn) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return -1;
-  cuuint64_t dims[2] = {(cuuint64_t)N, (cuuint64_t)M};
-  cuuint64_t strides[1] = {(cuuint64_t)(ldo * 2)};
-  cuuint32_t box[2] = {(cuuint32_t)bn, 32u};
-  cuuint32_t estr[2] = {1u, 1u};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box,
-                   estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                   CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : (int)r;
-}
-
 template <int BN, int AM, int BM, int GK, int GV, int NS>
 static int launch_stages(const CUtensorMap& ta, const CUtensorMap& tb, const GemmParams& p_in, dim3 grid,
                          cudaStream_t st) {
@@ -832,47 +748,14 @@ static int launch_stages(const CUtensorMap& ta, const CUtensorMap& tb, const Gem
     p.ktab_n = p.g.tpk > 0 ? p.g.ntaps : std::min(KTAB, (p.gK + step - 1) / step);
   }
   const int smem = ring + ((p.ktab_n + 3) & ~3) * 4 + BN * 4;
-  CUtensorMap tc = ta;
-  // TMA-store epilogue (smem staging + one tile store per warp) for plain bf16 row-major outputs.
-  // Measured on B200 it is slower than the direct 16-byte stores for these narrow tiles
-  // (CIFAR step 0.270 vs 0.263 ms; conv2 dgrad 25.7 vs 22.6 us): opt-in with ZNICZ_UMMA_TMA_STORE=1.
-  static int no_tma_store = -1;
-  if (no_tma_store < 0) { const char* e = getenv("ZNICZ_UMMA_TMA_STORE"); no_tma_store = (e && atoi(e)) ? 0 : 1; }
-  p.tma_store = 0;
-  if (!no_tma_store && p.out_bf16 && p.split_stride == 0 && !p.out_trans && p.beta == 0.f &&
-      (p.ldo % 8) == 0 && ((uintptr_t)p.out & 15) == 0 && 4 * 32 * BN * 2 <= ring - 1024 &&
-      p.mt <= 1) {      // (streamed tiles: the ring is busy with the next tile during the epilogue)
-    if (make_map_out(&tc, p.out, p.N, p.M, p.ldo, BN) == 0) p.tma_store = 1;
-  }
-  launch_k(gemm_umma_k<BN, AM, BM, GK, GV, NS>, grid, 192, smem, st, ta, tb, tc, p);
+  launch_k(gemm_umma_k<BN, AM, BM, GK, GV, NS>, grid, 192, smem, st, ta, tb, p);
   return (int)cudaGetLastError();
 }
 
 template <int BN, int AM, int BM, int GK, int GV>
-static int launch_cfg(const CUtensorMap& ta, const CUtensorMap& tb, const GemmParams& p_in, int splits,
+static int launch_cfg(const CUtensorMap& ta, const CUtensorMap& tb, const GemmParams& p, int splits,
                       cudaStream_t st) {
-  GemmParams p = p_in;
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("ZNICZ_UMMA_DBG"); dbg = e ? atoi(e) : 0; }
-    p.dbg = dbg;
-  }
-  const int m_tiles = (p.M + BLOCK_M - 1) / BLOCK_M;
-  const int mt = (AM == A_GATHER_K && p.mt > 1) ? p.mt : 1;
-  dim3 grid((p.N + BN - 1) / BN, (m_tiles + mt - 1) / mt, splits);
-  // Grids that leave one CTA (or none) per SM cannot hide the gather latency by co-residency:
-  // give those CTAs an 8-deep ring instead (asynchronous LDGSTS producers only, and only when
-  // the K loop is long enough to use it).
-  constexpr bool deep_ok = (GV == 2) && (8 * (A_BYTES + b_bytes<BN, BM>()) + 2048 <= 227 * 1024);
-  if constexpr (deep_ok) {
-    const long long ctas = (long long)grid.x * grid.y * grid.z;
-    const int kb = p.k_blocks_per_split;
-    // measured neutral on B200 for the CIFAR shapes (the per-k-block cost is not pipeline depth):
-    // opt-in with ZNICZ_UMMA_DEEP=1
-    static int deep = -1;
-    if (deep < 0) { const char* e = getenv("ZNICZ_UMMA_DEEP"); deep = e ? atoi(e) : 0; }
-    if (deep && ctas <= 160 && kb >= 8) return launch_stages<BN, AM, BM, GK, GV, 8>(ta, tb, p, grid, st);
-  }
+  dim3 grid((p.N + BN - 1) / BN, (p.M + BLOCK_M - 1) / BLOCK_M, splits);
   // Short reductions (K <= 4 k-blocks, e.g. a 5x5 first layer on 8 padded channels) in grids of
   // several waves: a 3-stage ring already holds almost the whole K and is small enough for a
   // third CTA per SM (ncu: these kernels are latency-bound at 15 % warp occupancy).
@@ -985,7 +868,7 @@ static int launch_fp8_bn(const CUtensorMap& ta, const CUtensorMap& tb, const Gem
     if (e != cudaSuccess) return (int)e;
     attr_set = true;
   }
-  launch_k(gemm_umma_k<BN, A_TMA_K, B_TMA_K, 0, 0, STAGES_DEFAULT, true>, grid, 192, smem, st, ta, tb, ta, p);
+  launch_k(gemm_umma_k<BN, A_TMA_K, B_TMA_K, 0, 0, STAGES_DEFAULT, true>, grid, 192, smem, st, ta, tb, p);
   return (int)cudaGetLastError();
 }
 // a [M][lda] e4m3, b [N][ldb] e4m3 (both K-major, ld % 16 == 0); alpha carries 1/(scale_a*scale_b)
@@ -1004,7 +887,7 @@ int launch_gemm_fp8(const void* a, long long lda, const void* b, long long ldb, 
   p.k_blocks_per_split = (K + 2 * BLOCK_K - 1) / (2 * BLOCK_K);
   p.out = out; p.out_bf16 = out_bf16; p.ldo = ldo; p.out_trans = 0;
   p.bias = bias; p.act = act; p.alpha = alpha; p.beta = 0.f; p.split_stride = 0;
-  p.gather_kind = G_NONE; p.mt = 1;
+  p.gather_kind = G_NONE;
   dim3 grid((N + bn - 1) / bn, (M + BLOCK_M - 1) / BLOCK_M, 1);
   switch (bn) {
     case 16: return launch_fp8_bn<16>(ta, tb, p, grid, st);
@@ -1018,24 +901,6 @@ static ConvGeomU geom(int N, int H, int W, int C, int OH, int OW, int F, int KY,
                       int PT, int PL, int vec) {
   ConvGeomU g{N, H, W, C, OH, OW, F, KY, KX, SY, SX, PT, PL, vec, 0, KY * KX, 0};
   return g;
-}
-// Tiles streamed per CTA (GemmParams::mt): only when the grid would otherwise need more than one
-// wave at two CTAs per SM, and never so many that fewer than one CTA per SM remains.
-static int pick_mt(int M, int N, int bn) {
-  const long long m_tiles = (M + BLOCK_M - 1) / BLOCK_M;
-  const long long n_tiles = (N + bn - 1) / bn;
-  // Measured on B200 (CIFAR step): with the epilogue of tile t overlapping the MMAs of tile t + 1
-  // (the "rounds" loop of the kernel) streaming 2 or 4 tiles per CTA is neutral (444.9 K / 445.3 K
-  // vs 442.7-447 K images/s); before that overlap existed it was slower (conv1 fprop 36 us vs
-  // 32.7 us). Independent CTAs already hide each other's prologues, so the mode stays opt-in
-  // (ZNICZ_UMMA_MT=2|4); a persistent scheduler with TMEM double buffering is the round-2 form.
-  static int forced = -1;
-  if (forced < 0) { const char* e = getenv("ZNICZ_UMMA_MT"); forced = e ? atoi(e) : 1; }
-  int mt = 1;
-  while (mt < forced && mt < 4 && bn * mt * 2 <= 256 && (m_tiles * n_tiles) / (mt * 2) >= 148 &&
-         m_tiles * n_tiles > 296)
-    mt *= 2;
-  return mt;
 }
 // Enable the tap-mode gather when the inner (channel) extent tiles a 64-wide reduction block.
 static bool set_tap_mode(ConvGeomU& g, int inner, bool dgrad) {
@@ -1082,13 +947,12 @@ int launch_conv_fprop_umma(const void* x, const void* w_lp, long long ldw, const
   p.bias = bias; p.act = act; p.alpha = 1.f; p.beta = 0.f; p.split_stride = 0;
   p.gsrc = (const __nv_bfloat16*)x; p.g = geom(N, H, W, C, OH, OW, F, KY, KX, SY, SX, PT, PL, C % 8 == 0);
   p.gather_kind = G_IM2COL; p.gK = Kw;
-  p.mt = pick_mt(p.M, p.N, bn);
   if (C % 64 == 0 && im2col_tma_enabled()) {
     // A operand by TMA im2col: window bases -PL .. W + upper_w, OW x OH of them
     CUtensorMap ti;
     if (make_map_im2col(&ti, x, N, H, W, C, -PL, -PT, (OW - 1) * SX + 1 - PL - W,
                         (OH - 1) * SY + 1 - PT - H, SX, SY, BLOCK_M) == 0) {
-      p.g.inner = C; p.mt = 1;
+      p.g.inner = C;
       ++g_im2col_launches;
       return launch_bn<A_IM2COL_K, B_TMA_K, G_IM2COL, 0>(bn, ti, tb, p, 1, st);
     }
@@ -1130,7 +994,6 @@ int launch_conv_dgrad_umma(const void* err_out, const void* wd_lp, long long ldc
   p.g = geom(N, H, W, C, OH, OW, F, KY, KX, SY, SX, PT, PL, F % 8 == 0);
   p.gather_kind = G_DGRAD; p.gK = Kd;
   p.dmul = (const __nv_bfloat16*)dmul; p.dact = dmul ? dact : 0;
-  p.mt = pick_mt(p.M, p.N, bn);
   if (F % 64 == 0 && SY == 1 && SX == 1 && im2col_tma_enabled()) {
     // unit stride: dgrad is a correlation of err_out with the flipped filter; W x H window bases
     // starting at -(K - 1 - pad) over the [N][OH][OW][F] tensor
@@ -1138,7 +1001,7 @@ int launch_conv_dgrad_umma(const void* err_out, const void* wd_lp, long long ldc
     const int lw = -(KX - 1 - PL), lh = -(KY - 1 - PT);
     if (make_map_im2col(&ti, err_out, N, OH, OW, F, lw, lh, W + lw - OW, H + lh - OH, 1, 1,
                         BLOCK_M) == 0) {
-      p.g.inner = F; p.mt = 1;
+      p.g.inner = F;
       ++g_im2col_launches;
       return launch_bn<A_IM2COL_K, B_TMA_MN, G_DGRAD, 0>(bn, ti, tb, p, 1, st);
     }
@@ -1180,22 +1043,6 @@ int launch_conv_wgrad_umma(const void* err_out, const void* x, float* partials, 
   p.bias = nullptr; p.act = 0; p.alpha = 1.f; p.beta = 0.f; p.split_stride = (long long)F * Kw;
   p.gsrc = (const __nv_bfloat16*)x; p.g = geom(N, H, W, C, OH, OW, F, KY, KX, SY, SX, PT, PL, C % 8 == 0);
   p.gather_kind = G_IM2COL; p.gK = Kw;
-  static int wg_tma = -1;
-  if (wg_tma < 0) { const char* e = getenv("ZNICZ_IM2COL_TMA_WGRAD"); wg_tma = (e && atoi(e)) ? 1 : 0; }
-  // (measured on the AlexNet shapes: 224-231 vs 231-249 TFLOP/s for the LDGSTS gather, which
-  // also delivers the bias row - so the single-CTA TMA form is opt-in; large layers take the
-  // 2-CTA kernel above)
-  if (wg_tma && C % 64 == 0 && im2col_tma_enabled()) {
-    // im2col operand by TMA, 64 pixels x 64 channels per box (no "ones" row here: the caller
-    // computes the bias gradient with the column-sum kernel when this returns 0)
-    CUtensorMap ti;
-    if (make_map_im2col(&ti, x, N, H, W, C, -PL, -PT, (OW - 1) * SX + 1 - PL - W,
-                        (OH - 1) * SY + 1 - PT - H, SX, SY, 64) == 0) {
-      p.g.inner = C;
-      ++g_im2col_launches;
-      return launch_bn<A_IM2COL_MN, B_TMA_MN, G_IM2COL, 0>(bn, ti, tb, p, splits, st);
-    }
-  }
   if (set_tap_mode(p.g, C, false)) {
     bool row = bias_parts != nullptr && (Kw % BLOCK_M) != 0;
     if (row) {

@@ -20,7 +20,7 @@ struct PoolGeom { int N, H, W, C, OH, OW, KY, KX, SY, SX; int act; int in_act; }
 template <typename T>
 __global__ void pool_forward_k(const T* __restrict__ in, T* __restrict__ out, int* __restrict__ offs,
                                PoolGeom g, int mode, const int* __restrict__ rng) {
-  pdl_entry();
+  pdl_wait();
   long long total = (long long)g.N * g.OH * g.OW * g.C;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
@@ -97,7 +97,7 @@ template <typename T>
 __global__ void pool_backward_max_k(const T* __restrict__ err_out, const int* __restrict__ offs,
                                     T* __restrict__ err_in, PoolGeom g, const T* __restrict__ yact,
                                     const T* __restrict__ xin) {
-  pdl_entry();
+  pdl_wait();
   long long total = (long long)g.N * g.H * g.W * g.C;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
@@ -121,7 +121,7 @@ __global__ void pool_backward_max_k(const T* __restrict__ err_out, const int* __
 template <typename T>
 __global__ void pool_backward_avg_k(const T* __restrict__ err_out, T* __restrict__ err_in, PoolGeom g,
                                     const T* __restrict__ yact, const T* __restrict__ xin) {
-  pdl_entry();
+  pdl_wait();
   long long total = (long long)g.N * g.H * g.W * g.C;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
@@ -149,7 +149,7 @@ __global__ void pool_backward_avg_k(const T* __restrict__ err_out, T* __restrict
 template <typename T>
 __global__ void pool_forward_vec_k(const T* __restrict__ in, T* __restrict__ out, int* __restrict__ offs,
                                    PoolGeom g, int mode) {
-  pdl_entry();
+  pdl_wait();
   const int C8 = g.C >> 3;
   const int total = g.N * g.OH * g.OW * C8;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -198,7 +198,7 @@ template <typename T>
 __global__ void pool_backward_vec_k(const T* __restrict__ err_out, const int* __restrict__ offs,
                                     T* __restrict__ err_in, PoolGeom g, int is_avg,
                                     const T* __restrict__ yact, const T* __restrict__ xin) {
-  pdl_entry();
+  pdl_wait();
   const int C8 = g.C >> 3;
   const int total = g.N * g.H * g.W * C8;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -250,7 +250,7 @@ __global__ void pool_backward_vec_k(const T* __restrict__ err_out, const int* __
 template <typename T, int half>
 __global__ void lrn_vec_k(const T* __restrict__ x, const T* __restrict__ ey, T* __restrict__ out,
                           int pixels, int C, float alpha, float beta, float k, int backward) {
-  pdl_entry();
+  pdl_wait();
   const int C8 = C >> 3;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= pixels * C8) return;
@@ -343,7 +343,7 @@ template <typename T, int KY, int KX, int SY, int SX>
 __global__ void __launch_bounds__(256)
 pool_forward_win_k(const T* __restrict__ in, T* __restrict__ out, int* __restrict__ offs, PoolGeom g,
                    int mode) {
-  pdl_entry();
+  pdl_wait();
   const int C8 = g.C >> 3;
   const int total = g.N * g.OH * g.OW * C8;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -401,100 +401,15 @@ pool_forward_win_k(const T* __restrict__ in, T* __restrict__ out, int* __restric
   st8(out + (size_t)i * 8, best);
 }
 
-template <typename T, int KY, int KX, int SY, int SX>
-__global__ void __launch_bounds__(256)
-pool_backward_win_k(const T* __restrict__ err_out, const int* __restrict__ offs, T* __restrict__ err_in,
-                    PoolGeom g, int is_avg, const T* __restrict__ yact, const T* __restrict__ xin) {
-  pdl_entry();
-  constexpr int NPY = (KY + SY - 1) / SY, NPX = (KX + SX - 1) / SX, NP = NPY * NPX;
-  const int C8 = g.C >> 3;
-  const int total = g.N * g.H * g.W * C8;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total) return;
-  const int cg = i % C8; int t = i / C8;
-  const int x = t % g.W; t /= g.W; const int y = t % g.H; const int n = t / g.H;
-  const int oy_hi = min(y / SY, g.OH - 1), ox_hi = min(x / SX, g.OW - 1);
-  const int oy_lo = (y - KY + 1 <= 0) ? 0 : (y - KY + SY) / SY;
-  const int ox_lo = (x - KX + 1 <= 0) ? 0 : (x - KX + SX) / SX;
-  const int self = i * 8;
-  Raw8<T> re[NP], ry[NP];
-  int4 oa[NP], ob[NP];
-  Raw8<T> rx;
-  rx.zero();
-  if (g.in_act) rx.load(xin + (size_t)i * 8);
-  // positions in ascending (oy, ox) order, like the generic kernel (same summation order)
-#pragma unroll
-  for (int jy = 0; jy < NPY; ++jy)
-#pragma unroll
-    for (int jx = 0; jx < NPX; ++jx) {
-      const int q = jy * NPX + jx;
-      const int oy = oy_hi - (NPY - 1 - jy), ox = ox_hi - (NPX - 1 - jx);
-      const bool ok = oy >= oy_lo && ox >= ox_lo;
-      re[q].zero(); ry[q].zero(); oa[q] = make_int4(-1, -1, -1, -1); ob[q] = oa[q];
-      if (ok) {
-        const int o = (((n * g.OH + oy) * g.OW + ox) * C8 + cg) * 8;
-        re[q].load(err_out + o);
-        if (g.act) ry[q].load(yact + o);
-        if (!is_avg) {
-          const int4* po = reinterpret_cast<const int4*>(offs + o);
-          oa[q] = po[0]; ob[q] = po[1];
-        }
-      }
-    }
-  float s[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) s[j] = 0.f;
-#pragma unroll
-  for (int jy = 0; jy < NPY; ++jy)
-#pragma unroll
-    for (int jx = 0; jx < NPX; ++jx) {
-      const int q = jy * NPX + jx;
-      const int oy = oy_hi - (NPY - 1 - jy), ox = ox_hi - (NPX - 1 - jx);
-      if (oy >= oy_lo && ox >= ox_lo) {
-        float e[8];
-        re[q].unpack(e);
-        if (g.act) {
-          float yv[8];
-          ry[q].unpack(yv);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) e[j] *= act_deriv(g.act, 0.f, yv[j]);
-        }
-        if (is_avg) {
-          const int hy = min(oy * SY + KY, g.H) - oy * SY;
-          const int hx = min(ox * SX + KX, g.W) - ox * SX;
-          const float inv = 1.f / (float)(hy * hx);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) s[j] += e[j] * inv;
-        } else {
-          const int of[8] = {oa[q].x, oa[q].y, oa[q].z, oa[q].w, ob[q].x, ob[q].y, ob[q].z, ob[q].w};
-#pragma unroll
-          for (int j = 0; j < 8; ++j) if (of[j] == self + j) s[j] += e[j];
-        }
-      }
-    }
-  if (g.in_act) {
-    float xv[8];
-    rx.unpack(xv);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) s[j] *= act_deriv(g.in_act, 0.f, xv[j]);
-  }
-  st8(err_in + (size_t)i * 8, s);
-}
-
-// Per-kernel ncu timing on B200 (CIFAR layers, bf16): the fixed-window FORWARD kernel is faster
-// than the generic one (3.7-4.2 us vs 5.2-5.9 us, pool1 7.1 vs 7.7 us) and is the default; the
-// fixed-window BACKWARD kernel is slower (pool1 27 us vs 17.5 us: 4 positions x (err + offsets +
-// output) held in registers costs more occupancy than the serialised round trips it removes)
-// and stays opt-in (ZNICZ_POOL_WIN_BWD=1). ZNICZ_POOL_WIN=0 disables both.
-static bool pool_win_enabled(bool backward) {
-  static int fwd = -1, bwd = -1;
-  if (fwd < 0) {
-    const char* e = getenv("ZNICZ_POOL_WIN");
-    fwd = (e && atoi(e) == 0) ? 0 : 1;
-    const char* b = getenv("ZNICZ_POOL_WIN_BWD");
-    bwd = (fwd && b && atoi(b) != 0) ? 1 : 0;
-  }
-  return backward ? bwd != 0 : fwd != 0;
+// Per-kernel ncu timing on B200 (CIFAR layers, bf16): the fixed-window forward kernel is faster
+// than the generic one (3.7-4.2 us vs 5.2-5.9 us, pool1 7.1 vs 7.7 us) and is the default;
+// ZNICZ_POOL_WIN=0 selects the generic one. A fixed-window backward kernel was slower (pool1 27 us
+// vs 17.5 us: 4 positions x (err + offsets + output) held in registers cost more occupancy than
+// the serialised round trips it removed), so backward always takes the generic kernel.
+static bool pool_win_enabled() {
+  static int on = -1;
+  if (on < 0) { const char* e = getenv("ZNICZ_POOL_WIN"); on = (e && atoi(e) == 0) ? 0 : 1; }
+  return on != 0;
 }
 
 void launch_pool_forward(const void* in, void* out, int* offs, int N, int H, int W, int C, int OH, int OW,
@@ -506,10 +421,10 @@ void launch_pool_forward(const void* in, void* out, int* offs, int N, int H, int
       (((uintptr_t)in | (uintptr_t)out | (uintptr_t)offs) & 15) == 0) {
     int gridv = cdiv(total / 8, 256);
     typedef __nv_bfloat16 bf;
-    if (pool_win_enabled(false) && KY == 3 && KX == 3 && SY == 2 && SX == 2) {
+    if (pool_win_enabled() && KY == 3 && KX == 3 && SY == 2 && SX == 2) {
       if (bf16) launch_k(pool_forward_win_k<bf, 3, 3, 2, 2>, gridv, 256, 0, st, (const bf*)in, (bf*)out, offs, g, mode);
       else launch_k(pool_forward_win_k<float, 3, 3, 2, 2>, gridv, 256, 0, st, (const float*)in, (float*)out, offs, g, mode);
-    } else if (pool_win_enabled(false) && KY == 2 && KX == 2 && SY == 2 && SX == 2) {
+    } else if (pool_win_enabled() && KY == 2 && KX == 2 && SY == 2 && SX == 2) {
       if (bf16) launch_k(pool_forward_win_k<bf, 2, 2, 2, 2>, gridv, 256, 0, st, (const bf*)in, (bf*)out, offs, g, mode);
       else launch_k(pool_forward_win_k<float, 2, 2, 2, 2>, gridv, 256, 0, st, (const float*)in, (float*)out, offs, g, mode);
     } else if (bf16) launch_k(pool_forward_vec_k<__nv_bfloat16>, gridv, 256, 0, st, (const __nv_bfloat16*)in, (__nv_bfloat16*)out, offs, g, mode);
@@ -529,13 +444,7 @@ void launch_pool_backward(const void* err_out, const int* offs, void* err_in, in
   if (C % 8 == 0 && total < (1LL << 31) &&
       (((uintptr_t)err_out | (uintptr_t)err_in | (uintptr_t)offs | (uintptr_t)yact | (uintptr_t)xin) & 15) == 0) {
     int gridv = cdiv(total / 8, 256);
-    if (pool_win_enabled(true) && KY == 3 && KX == 3 && SY == 2 && SX == 2) {
-      if (bf16) launch_k(pool_backward_win_k<bf, 3, 3, 2, 2>, gridv, 256, 0, st, (const bf*)err_out, offs, (bf*)err_in, g, is_avg, (const bf*)yact, (const bf*)xin);
-      else launch_k(pool_backward_win_k<float, 3, 3, 2, 2>, gridv, 256, 0, st, (const float*)err_out, offs, (float*)err_in, g, is_avg, (const float*)yact, (const float*)xin);
-    } else if (pool_win_enabled(true) && KY == 2 && KX == 2 && SY == 2 && SX == 2) {
-      if (bf16) launch_k(pool_backward_win_k<bf, 2, 2, 2, 2>, gridv, 256, 0, st, (const bf*)err_out, offs, (bf*)err_in, g, is_avg, (const bf*)yact, (const bf*)xin);
-      else launch_k(pool_backward_win_k<float, 2, 2, 2, 2>, gridv, 256, 0, st, (const float*)err_out, offs, (float*)err_in, g, is_avg, (const float*)yact, (const float*)xin);
-    } else if (bf16) launch_k(pool_backward_vec_k<bf>, gridv, 256, 0, st, (const bf*)err_out, offs, (bf*)err_in, g, is_avg, (const bf*)yact, (const bf*)xin);
+    if (bf16) launch_k(pool_backward_vec_k<bf>, gridv, 256, 0, st, (const bf*)err_out, offs, (bf*)err_in, g, is_avg, (const bf*)yact, (const bf*)xin);
     else launch_k(pool_backward_vec_k<float>, gridv, 256, 0, st, (const float*)err_out, offs, (float*)err_in, g, is_avg, (const float*)yact, (const float*)xin);
     return;
   }
@@ -554,7 +463,7 @@ void launch_pool_backward(const void* err_out, const int* offs, void* err_in, in
 template <typename T>
 __global__ void lrn_forward_k(const T* __restrict__ x, T* __restrict__ y, long long pixels, int C,
                               int half, float alpha, float beta, float k) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= pixels * C) return;
   int c = (int)(i % C);
@@ -570,7 +479,7 @@ template <typename T>
 __global__ void lrn_backward_k(const T* __restrict__ ey, const T* __restrict__ x, T* __restrict__ eh,
                                long long pixels, int C, int half, float alpha, float beta, float k,
                                int in_act) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= pixels * C) return;
   int c = (int)(i % C);

@@ -14,7 +14,7 @@ namespace zn {
 template <typename T>
 __global__ void space_to_depth_k(const T* __restrict__ x, __nv_bfloat16* __restrict__ xs, int N, int H, int W,
                                  int C, int s, int pad_t, int pad_l, int Hs, int Ws, int Cp) {
-  pdl_entry();
+  pdl_wait();
   const long long total = (long long)N * Hs * Ws * Cp;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -36,7 +36,7 @@ __global__ void space_to_depth_k(const T* __restrict__ x, __nv_bfloat16* __restr
 // fp32 master weights [F][ky][kx][C] -> bf16 [F][kyp][kxp][Cp] in the space-to-depth tap order
 __global__ void s2d_pack_weights_k(const float* __restrict__ w, __nv_bfloat16* __restrict__ ws, int F, int ky,
                                    int kx, int C, int s, int kyp, int kxp, int Cp) {
-  pdl_entry();
+  pdl_wait();
   const long long total = (long long)F * kyp * kxp * Cp;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -58,7 +58,7 @@ __global__ void s2d_pack_weights_k(const float* __restrict__ w, __nv_bfloat16* _
 // gradient partials in the space-to-depth layout [parts][Fr][kyp][kxp][Cp] -> [parts][F][ky][kx][C]
 __global__ void s2d_unpack_grad_k(const float* __restrict__ gs, float* __restrict__ g, int parts, int F, int Fr,
                                   int ky, int kx, int C, int s, int kyp, int kxp, int Cp) {
-  pdl_entry();
+  pdl_wait();
   const long long total = (long long)parts * F * ky * kx * C;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {

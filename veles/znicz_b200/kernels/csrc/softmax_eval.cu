@@ -12,7 +12,7 @@ namespace zn {
 template <typename T>
 __global__ void softmax_rows_k(const T* __restrict__ in, float* __restrict__ out,
                                int* __restrict__ max_idx, int rows, int cols) {
-  pdl_entry();
+  pdl_wait();
   int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= rows) return;
   const T* r = in + (size_t)warp * cols;
@@ -39,7 +39,7 @@ __global__ void evaluate_softmax_k(const float* __restrict__ y, const int* __res
                                    const float* __restrict__ bp, int rows, int cols,
                                    int* __restrict__ n_err, int* __restrict__ confusion,
                                    float* __restrict__ max_err_sum) {
-  pdl_entry();
+  pdl_wait();
   int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= rows) return;
   int batch = (int)bp[0]; float mult = bp[1];
@@ -71,7 +71,7 @@ __global__ void evaluate_mse_k(const TY* __restrict__ y, const TY* __restrict__ 
                                TE* __restrict__ err, const float* __restrict__ bp, int rows, int cols,
                                const float* __restrict__ denorm_mul, int root,
                                float* __restrict__ metrics, float* __restrict__ mse) {
-  pdl_entry();
+  pdl_wait();
   int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= rows) return;
   int batch = (int)bp[0]; float mult = bp[1];
@@ -105,7 +105,7 @@ template <typename TY>
 __global__ void mse_find_closest_k(const TY* __restrict__ y, const float* __restrict__ class_targets,
                                    const int* __restrict__ labels, const float* __restrict__ bp,
                                    int rows, int cols, int n_targets, int* __restrict__ n_err) {
-  pdl_entry();
+  pdl_wait();
   int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= rows || warp >= (int)bp[0]) return;
   const TY* r = y + (size_t)warp * cols;

@@ -11,7 +11,7 @@ namespace zn {
 __global__ void som_winners_k(const float* __restrict__ x, const float* __restrict__ w,
                               int* __restrict__ argmins, int* __restrict__ winners, int neurons,
                               int len, int count_winners) {
-  pdl_entry();
+  pdl_wait();
   const int s = blockIdx.x;
   const float* xs = x + (size_t)s * len;
   float best = 3.0e38f; int bi = 0x7fffffff;
@@ -47,7 +47,7 @@ __global__ void som_winners_k(const float* __restrict__ x, const float* __restri
 __global__ void som_update_k(const float* __restrict__ x, float* __restrict__ w,
                              const float* __restrict__ coords, const int* __restrict__ argmins,
                              int batch, int neurons, int len, float sigma, float gmult) {
-  pdl_entry();
+  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= neurons * len) return;
   const int n = i / len, k = i - n * len;
@@ -79,7 +79,7 @@ __global__ void som_update_k(const float* __restrict__ x, float* __restrict__ w,
 __global__ void som_split_k(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, int rows,
                             int len, int kp, long long ld, long long part_stride, int pattern,
                             float* __restrict__ norm_out) {
-  pdl_entry();
+  pdl_wait();
   const int row = blockIdx.x;
   if (row >= rows) return;
   const float* s = src + (size_t)row * len;
@@ -111,7 +111,7 @@ __global__ void som_split_k(const float* __restrict__ src, __nv_bfloat16* __rest
 __global__ void som_argmin_k(const float* __restrict__ dots, const float* __restrict__ wnorm,
                              int* __restrict__ argmins, int* __restrict__ winners, int neurons,
                              int count_winners) {
-  pdl_entry();
+  pdl_wait();
   const int s = blockIdx.x;
   const float* d = dots + (size_t)s * neurons;
   float best = 3.0e38f; int bi = 0x7fffffff;
@@ -147,7 +147,7 @@ __global__ void som_argmin_k(const float* __restrict__ dots, const float* __rest
 __global__ void som_gravity_split_k(const float* __restrict__ coords, const int* __restrict__ argmins,
                                     __nv_bfloat16* __restrict__ dst, float* __restrict__ rowsum,
                                     int batch, int bp, float sigma) {
-  pdl_entry();
+  pdl_wait();
   const int n = blockIdx.x;
   const float cx = coords[2 * n], cy = coords[2 * n + 1];
   const float inv = -1.f / (2.f * sigma * sigma);
@@ -178,7 +178,7 @@ __global__ void som_gravity_split_k(const float* __restrict__ coords, const int*
 // w[n][k] += gmult * (M[n][k] - rowsum[n] * w[n][k])
 __global__ void som_apply_k(float* __restrict__ w, const float* __restrict__ m,
                             const float* __restrict__ rowsum, long long total, int len, float gmult) {
-  pdl_entry();
+  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const float wv = w[i];

@@ -34,7 +34,7 @@ __device__ __forceinline__ void split_store(const SplitDst& d, long long row, in
 // of dgrad and the row-stacked operand of wgrad from the same err_output)
 __global__ void split_parts_k(const float* __restrict__ src, long long rows, int len, int kmax,
                               SplitDst a, SplitDst b) {
-  pdl_entry();
+  pdl_wait();
   const long long total = rows * kmax;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -51,7 +51,7 @@ __global__ void split_parts_k(const float* __restrict__ src, long long rows, int
 // conv weights fp32 [F][taps][C] -> the dgrad operand [taps][nparts * Fp][Cp] (parts along F)
 __global__ void split_conv_wt_k(const float* __restrict__ w, __nv_bfloat16* __restrict__ dst, int F,
                                 int taps, int C, int Fp, int Cp, int nparts, int pattern) {
-  pdl_entry();
+  pdl_wait();
   const long long total = (long long)taps * Fp * Cp;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {

@@ -117,10 +117,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void*
                "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
                : "memory");
 }
-__device__ __forceinline__ void tma_store_commit_and_wait_read() {
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-}
 
 // ------------------------------------------------------------------ tcgen05
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {

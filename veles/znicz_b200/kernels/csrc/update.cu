@@ -110,7 +110,7 @@ __global__ void fused_update_k(float* __restrict__ w, GradSources gs, float* __r
                                const float* __restrict__ hyper, const float* __restrict__ col_sums,
                                int flags, int is_bias, long long size, int rows, int cols,
                                ShadowSpec sh, PeerSync ps) {
-  pdl_entry();
+  pdl_wait();
   __shared__ uint32_t s_epoch;
   uint32_t epoch = 0;
   if (MULTI) {
@@ -190,7 +190,7 @@ __global__ void fused_update_k(float* __restrict__ w, GradSources gs, float* __r
 // column sums of W (pre-update) for the orthogonality regulariser: out[col] = sum_row w[row, col]
 __global__ void col_sums_k(const float* __restrict__ w, float* __restrict__ out, int rows, int cols,
                            int transposed) {
-  pdl_entry();
+  pdl_wait();
   // logical matrix [rows=Y][cols=H]; when transposed the storage is [H][Y]
   int col = blockIdx.x * blockDim.y + threadIdx.y;
   if (col >= cols) return;
@@ -204,7 +204,7 @@ __global__ void col_sums_k(const float* __restrict__ w, float* __restrict__ out,
 // shadow refresh without an update step (initialisation, rollback, weights from a snapshot)
 __global__ void refresh_shadows_k(const float* __restrict__ w, long long size, int rows, int cols,
                                   ShadowSpec sh) {
-  pdl_entry();
+  pdl_wait();
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long stride = (long long)gridDim.x * blockDim.x;
   for (; i < size; i += stride) {
@@ -636,7 +636,6 @@ __device__ __forceinline__ void multi_reduce_bcast(const TensorDesc& d, int tile
 __global__ void __launch_bounds__(256, 4)
 multi_update_k(const TensorDesc* __restrict__ table, int n, int total_tiles, int has_ortho,
                PeerSync ps, GridSync gsync, RedBufs rb) {
-  pdl_trigger();
   __shared__ uint32_t s_epoch;
   __shared__ TensorDesc s_table[MU_MAX_TENSORS];     // the whole table: no dependent global loads
   const bool multi = ps.nranks > 1;
